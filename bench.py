@@ -80,6 +80,8 @@ def parse():
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only: skip the host-input arm")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--with-optimizer", action="store_true", help="also run vlbert_b200.optim.FusedAdamW (+ global-norm clip) in every step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss and the parameter gradients of the last timed step as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -295,7 +297,7 @@ def cpu_baseline(w, p_drop, steps=1, warmup=1, batch=None, threads=None):
         if i >= warmup:
             times.append(time.perf_counter() - t0)
     dt = sum(times) / len(times)
-    return {"value": batch / dt, "unit": "samples/s", "cores": cores, "kind": "port",
+    return {"value": batch / dt, "unit": "samples/s", "cores": cores, "kind": "port", "steps": steps, "warmup": warmup,
             "sample": "%d timed step(s) after %d warm-up of the FULL workload (batch %d, %d layers, S=%d, dropout %.2g through torch's generator), "
                       "fp32, torch CPU ops on %d threads" % (steps, warmup, batch, w["layers"], seq_len(w), p_drop, cores),
             "ms_per_step": dt * 1e3}
@@ -330,7 +332,7 @@ def gpu_eager_baseline(w, p_drop, device, steps=3, warmup=2):
             e1.record()
             torch.cuda.synchronize()
             ms = e0.elapsed_time(e1) / steps
-            out[name] = {"ms_per_step": ms, "samples_per_s": w["batch"] / ms * 1e3,
+            out[name] = {"ms_per_step": ms, "steps": steps, "warmup": warmup, "samples_per_s": w["batch"] / ms * 1e3,
                          "model_flops_tflops": w["batch"] * encoder_flop_per_sample(w) / ms / 1e9}
         except Exception as e:  # noqa
             out[name] = {"error": str(e)[:200]}
@@ -347,13 +349,13 @@ def run_reference(args):
     w = WORKLOADS[args.config]
     if args.batch:
         w = dict(w, batch=args.batch)
-    cb = cpu_baseline(w, args.dropout, steps=max(1, min(args.steps, 2)), warmup=1)
+    cb = cpu_baseline(w, args.dropout, steps=args.steps, warmup=args.warmup)
     line = {"impl": "reference", "metric": "samples/sec VL-BERT-base fwd+bwd", "value": cb["value"], "unit": "samples/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "%s: %s (S=%d), batch %d, fwd+bwd, dropout %.2g, CPU fp32 (the reference's module graph, oracle port)"
                                    % (w["name"], w["what"], seq_len(w), w["batch"], args.dropout)},
-            "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")},
+            "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "steps", "warmup", "sample")},
             "e2e": {"value": cb["value"], "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
 
@@ -482,7 +484,7 @@ class Runner(object):
             sampler.active = True
         e0.record()
         for _ in range(steps):
-            self.step(self.dev_inputs)
+            self.last_loss = self.step(self.dev_inputs)
         e1.record()
         self.barrier()
         if sampler:
@@ -553,6 +555,27 @@ def optimizer_roofline(run, pk, iters=20):
             "frac": gbs / pk["hbm_gbs"] if pk.get("hbm_gbs") else None, "launches_per_step": 2}
 
 
+DUMP_SAMPLE = 1 << 16      # gradient elements kept per parameter tensor (a fixed seeded sample of larger ones)
+
+
+def dump_outputs(run, out_dir):
+    """What the last timed step handed its caller: the loss and every parameter gradient, as float32 .npy files.  Of a gradient
+    larger than DUMP_SAMPLE elements only the elements at DUMP_SAMPLE fixed flat indices are written (the sorted head of
+    randperm(numel) seeded with the parameter's position in named_parameters()), which keeps the whole dump well under 64 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), run.last_loss.detach().float().cpu().numpy())
+    for i, (name, p) in enumerate(run.model.named_parameters()):
+        if p.grad is None:
+            continue
+        g = p.grad.detach().float().reshape(-1)
+        base = os.path.join(out_dir, "grad." + name)
+        if g.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(g.numel(), generator=torch.Generator().manual_seed(i))[:DUMP_SAMPLE].sort().values
+            g = g[idx.to(g.device)]
+        np.save(base + ".npy", g.cpu().numpy())
+
+
 def workload_text(w, B, p_drop, with_opt):
     return "%s: %s (S=%d), batch %d per GPU, fwd+bwd in training mode (dropout p=%.2g at every reference site), %s%s" % (
         w["name"], w["what"], seq_len(w), B, p_drop,
@@ -618,6 +641,8 @@ def main():
     if sampler:
         sampler.start()
     ms = run.timed(args.steps, args.warmup, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(run, args.dump_outputs)
     launches = run.launches_per_step()
 
     # ---------------- end-to-end arm: pinned host inputs -> H2D -> step -> loss read back ----------------
@@ -727,7 +752,7 @@ def main():
                 r2 = Runner(wo, a2, dev, rank, world, dist)
                 ps = 2
                 pm2, pw2, pc2 = r2.profile(ps)
-                n_steps = 10 if c != 5 else 5
+                n_steps = args.steps
                 ms2 = r2.timed(n_steps, 3)
                 roof2 = r2.roofline(pm2, pw2, ms2, pk, pk_kind, ps)
                 unit = "images/s" if wo["head"] == "frontend" else ("sequences/s" if c == 4 else "samples/s")
@@ -745,10 +770,10 @@ def main():
                 torch.cuda.empty_cache()
         line["other_configs"] = others
     if world == 1 and not args.no_gpu_eager:
-        line["gpu_eager_baseline"] = gpu_eager_baseline(w, args.dropout, dev)
+        line["gpu_eager_baseline"] = gpu_eager_baseline(w, args.dropout, dev, steps=args.steps)
     if not args.no_cpu_baseline and world == 1:
         cb = cpu_baseline(w, args.dropout)
-        line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")}
+        line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "steps", "warmup", "sample")}
     print(json.dumps(line))
     sys.stdout.flush()
     if dist is not None:

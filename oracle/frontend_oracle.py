@@ -8,8 +8,8 @@ Follows (reference file:line):
   _ROIAlign                     common/lib/roi_pooling/roi_align.py:11-43  (via oracle/roi_align_oracle.c)
 
 It is a function of a reference-format state_dict (keys `backbone.*`, `roi_head_feature_extractor.*`,
-`obj_downsample.1.*`), so it is pinned two ways: against the live reference module in this container
-(tests/test_oracle_vs_reference.py) and by the committed fixture tests/golden/fastrcnn_e2e.npz that
+`obj_downsample.1.*`), so it is pinned two ways: against the reference module's outputs with instance masks
+(tests/test_oracle_vs_reference.py, tests/golden/reference_parity.npz) and by the committed fixture tests/golden/fastrcnn_e2e.npz that
 oracle/make_golden.py wrote from the reference.  BatchNorm is the eval-mode (frozen statistics) map, the
 only mode the reference runs the backbone in (common/fast_rcnn.py:122-126, FastRCNN.bn_eval).
 
@@ -18,7 +18,8 @@ weights, each conv+BN(+ReLU) output, RoIAlign output, the region operand and the
 backward (straight-through).  ReLU networks amplify forward rounding into gradient error (a pre-activation within
 rounding distance of 0 flips its mask and moves that element's gradient by 100%: relative L2 error ~ sqrt(fraction
 flipped)), so the fp32 graph bounds the CUDA path's gradients only loosely; the bf16-storage graph has the same masks
-and bounds them tightly.  tests/test_gpu_frontend.py uses both.
+and bounds them tightly.  tests/test_gpu_frontend.py uses both.  The graph computes in the dtype of its inputs (fp32, or
+fp64 between the bf16 storage points for a comparator that does not depend on the host's summation order).
 
 Only tests/, __graft_entry__.smoke() and bench.py's CPU legs may import this module.
 """
@@ -39,11 +40,11 @@ LAYERS = {50: (3, 4, 6), 101: (3, 4, 23), 152: (3, 8, 36)}
 class _RoundBF16(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x):
-        return x.to(torch.bfloat16).float()
+        return x.to(torch.bfloat16).to(x.dtype)
 
     @staticmethod
     def backward(ctx, g):
-        return g.to(torch.bfloat16).float()
+        return g.to(torch.bfloat16).to(g.dtype)
 
 
 def _q(storage):
@@ -95,13 +96,13 @@ class _RoIAlign(torch.autograd.Function):
     def forward(ctx, feat, rois, ph, pw, scale, sr):
         ctx.save_for_backward(rois)
         ctx.cfg = (ph, pw, scale, sr, tuple(feat.shape))
-        return torch.from_numpy(_roi.roi_align_forward(feat.detach().numpy(), rois.numpy(), scale, ph, pw, sr))
+        return torch.from_numpy(_roi.roi_align_forward(feat.detach().numpy(), rois.numpy(), scale, ph, pw, sr)).to(feat.dtype)
 
     @staticmethod
     def backward(ctx, g):
         (rois,) = ctx.saved_tensors
         ph, pw, scale, sr, (N, C, H, W) = ctx.cfg
-        return torch.from_numpy(_roi.roi_align_backward(g.contiguous().numpy(), rois.numpy(), scale, ph, pw, N, C, H, W, sr)), \
+        return torch.from_numpy(_roi.roi_align_backward(g.contiguous().numpy(), rois.numpy(), scale, ph, pw, N, C, H, W, sr)).to(g.dtype), \
             None, None, None, None, None
 
 

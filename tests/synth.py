@@ -118,3 +118,34 @@ def adamw_case(seed=5):
     groups = [dict(idx=[0, 2], lr=2e-3, weight_decay=0.01), dict(idx=[1], lr=1e-3, weight_decay=0.0)]
     lr_scale = [0.25, 0.5, 0.75, 1.0]
     return params, grads, groups, lr_scale
+
+
+def fake_hf_checkpoint(kind, H=64, L=2, I=128, vocab=120, max_pos=40):
+    """a state_dict with HuggingFace BERT (old TF-style gamma/beta names, cls.* heads) or RoBERTa (roberta.*, lm_head.*, one
+    token type) key names, random values"""
+    g = torch.Generator().manual_seed(7 if kind == "bert" else 8)
+    r = lambda *s: torch.randn(*s, generator=g)
+    pre = "bert." if kind == "bert" else "roberta."
+    ln_w, ln_b = ("gamma", "beta") if kind == "bert" else ("weight", "bias")
+    sd = {pre + "embeddings.word_embeddings.weight": r(vocab, H), pre + "embeddings.position_embeddings.weight": r(max_pos, H),
+          pre + "embeddings.token_type_embeddings.weight": r(2 if kind == "bert" else 1, H),
+          pre + "embeddings.LayerNorm." + ln_w: r(H), pre + "embeddings.LayerNorm." + ln_b: r(H),
+          pre + "embeddings.position_ids": torch.arange(max_pos)[None],                       # unexpected key
+          pre + "pooler.dense.weight": r(H, H), pre + "pooler.dense.bias": r(H)}
+    for l in range(L):
+        q = pre + "encoder.layer.%d." % l
+        for n, shp in (("attention.self.query", (H, H)), ("attention.self.key", (H, H)), ("attention.self.value", (H, H)),
+                       ("attention.output.dense", (H, H)), ("intermediate.dense", (I, H)), ("output.dense", (H, I))):
+            sd[q + n + ".weight"], sd[q + n + ".bias"] = r(*shp), r(shp[0])
+        for n in ("attention.output.LayerNorm", "output.LayerNorm"):
+            sd[q + n + "." + ln_w], sd[q + n + "." + ln_b] = r(H), r(H)
+    if kind == "bert":
+        sd.update({"cls.seq_relationship.weight": r(2, H), "cls.seq_relationship.bias": r(2),
+                   "cls.predictions.bias": r(vocab), "cls.predictions.transform.dense.weight": r(H, H),
+                   "cls.predictions.transform.dense.bias": r(H), "cls.predictions.transform.LayerNorm.gamma": r(H),
+                   "cls.predictions.transform.LayerNorm.beta": r(H), "cls.predictions.decoder.weight": r(vocab, H)})
+    else:
+        sd.update({"lm_head.bias": r(vocab), "lm_head.dense.weight": r(H, H), "lm_head.dense.bias": r(H),
+                   "lm_head.layer_norm.weight": r(H), "lm_head.layer_norm.bias": r(H), "lm_head.decoder.weight": r(vocab, H)})
+    sd["some.other.tensor"] = r(3)
+    return sd

@@ -1,12 +1,12 @@
-"""CPU, build container only (skipped where /root/reference is absent): the reference's OWN training loop --
+"""CPU.  The first test needs the reference tree (it is skipped where the tree is absent): the reference's OWN training loop --
 common/trainer.py:train (:56-197: net.train(), forward, loss.mean(), backward, LR-scheduler step, clip_grad_norm_,
 optimizer.step(), zero_grad, metrics.update) -- driven for several optimisation steps on
 pretrain.modules.ResNetVLBERTForPretraining built from cfgs/pretrain/base_prec_4x16G_fp32.yaml (2 layers, synthetic
 loader: BASELINE config 1, "plumbing"), once untouched and once after vlbert_b200.dropin.install().  The loss trajectory,
 the metrics the loop accumulates and the final weights have to agree.
 
-What is a stand-in here and why: there is no GPU in the build container and no /root/reference on the GPU box, so the two
-cannot meet in one process.  The kernels are therefore replaced by the fp32 torch stand-ins of tests/cpu_shim.py (this
+What is a stand-in here and why: the reference tree and a GPU are not expected on the same machine, so the two cannot meet
+in one process.  The kernels are therefore replaced by the fp32 torch stand-ins of tests/cpu_shim.py (this
 checks every decision of the Python layer under the real loop: train()/eval() switching, parameter registration seen by the
 optimizer and by clip_grad_norm_, in-place updates of the weights the fused path caches, gradient accumulation), `to_cuda`
 (common/trainer.py:42-53) is replaced by the identity, and dropout probabilities are 0 (the stand-ins have no Philox masks;
@@ -22,7 +22,6 @@ import torch
 
 import ref_shim
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 
 STEPS_PER_EPOCH, EPOCHS = 3, 2
 
@@ -70,6 +69,7 @@ class _Recorder(object):
         self.losses.append(float(p.locals["loss"].detach()))
 
 
+@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 @pytest.mark.parametrize("accumulate", [1, 2])
 def test_reference_trainer_loop_runs_identically_on_the_dropin(tmp_path, monkeypatch, capsys, accumulate):
     ref_shim.install()
@@ -187,9 +187,7 @@ def test_dropin_module_survives_torch_ddp_wrapper_and_the_native_reducer(monkeyp
         return {k: p.grad.clone() for k, p in mod.named_parameters() if p.grad is not None}
 
     g0 = grads(model)
-    os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-    os.environ.setdefault("MASTER_PORT", "29571")
-    dist.init_process_group("gloo", rank=0, world_size=1)
+    dist.init_process_group("gloo", store=dist.HashStore(), rank=0, world_size=1)      # in-process store: no TCP port to collide on
     try:
         wrapped = torch.nn.parallel.DistributedDataParallel(model)
         for _ in range(2):
