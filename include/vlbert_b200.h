@@ -322,6 +322,29 @@ int vlb_mlm_ce_forward(const void* logits_bf16, int ld, int V, const int32_t* la
 int vlb_mlm_ce_backward(void* logits_bf16, int ld, int V, const int32_t* lab, const int32_t* count, int rows, const float* lse,
                         const float* gscale, void* stream);
 
+/* ---- masked visual region classification (MVRC) loss head ----------------------------------------------
+ * Replaces, for the LOSS path, VisualLinguisticBertMVRCHead + soft_cross_entropy of the pre-training task
+ * (common/visual_linguistic_bert.py:473-502; common/utils/misc.py:124-151; pretrain/modules/resnet_vlbert_for_pretraining.py:
+ * 191-203).  A region row is valid when its fp32 soft target sums to 1 within 0.1; only those (~15 %) enter the loss.
+ *   vlb_soft_target_rows: targets f32 [n, C] (row stride ld_t, rows only 4-byte aligned is fine): arg[row] (int64) = first
+ *                       index of the row's maximum target if |sum - 1| < 0.1, else -1.  Feed arg to vlb_label_compact with
+ *                       ignore_index = -1: idx = valid rows (ascending), lab = their target arg-max, count = their number.
+ *   (caller: gather those rows with vlb_gather_rows; transform GEMM (+ bias + erf-GELU, act 1) and classifier GEMM with
+ *    vlb_gemm_bf16 on `rows` rows into bf16 logits [rows, ld], ld = C padded to 8, padding columns biased to -30000)
+ *   vlb_soft_ce_forward: per compacted row < count, reading targets[idx[row]] in place: lse[row] = log-sum-exp of the first
+ *                       C logits; row_loss[row] = S lse - sum_c t_c x_c (= -sum_c t_c log_softmax(x)_c, S = sum_c t_c);
+ *                       correct[0] += (logit arg-max == lab[row])  (what MVRCAccuracy counts).  Rows >= count: row_loss 0.
+ *   vlb_soft_ce_backward: overwrites the logits IN PLACE with d loss / d logits = (S softmax(x) - t) * w[row], w = the
+ *                       per-row DEVICE weight d loss / d row_loss (rows >= count and padding columns: 0).
+ * No host synchronisation: count stays on the device.
+ */
+int vlb_soft_target_rows(const float* targets, int n, int C, int ld_t, int64_t* arg, void* stream);
+int vlb_soft_ce_forward(const void* logits_bf16, int ld, int C, const float* targets, int ld_t, const int32_t* idx,
+                        const int32_t* lab, const int32_t* count, int rows, float* lse, float* row_loss, int32_t* correct,
+                        void* stream);
+int vlb_soft_ce_backward(void* logits_bf16, int ld, int C, const float* targets, int ld_t, const int32_t* idx,
+                         const int32_t* count, int rows, const float* lse, const float* w, void* stream);
+
 /* ---- optimizer step after the path (SURVEY 8(f) rank 2) ---------------------------------------------
  * Replaces AdamW.step (common/nlp/bert/optimization.py:129-187: Adam moments, bias-corrected step size, decoupled weight decay
  * applied AFTER the update) and torch.nn.utils.clip_grad_norm_ of the trainer (common/trainer.py:139-147) for all parameter

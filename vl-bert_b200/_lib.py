@@ -86,6 +86,9 @@ def _declare(lib):
     decl("vlb_label_compact", [P, I, L, P, P, I, P, P])
     decl("vlb_mlm_ce_forward", [P, I, I, P, P, I, P, P, P, P])
     decl("vlb_mlm_ce_backward", [P, I, I, P, P, I, P, P, P])
+    decl("vlb_soft_target_rows", [P, I, I, I, P, P])
+    decl("vlb_soft_ce_forward", [P, I, I, P, I, P, P, P, I, P, P, P, P])
+    decl("vlb_soft_ce_backward", [P, I, I, P, I, P, P, I, P, P, P])
     decl("vlb_layer_dropout_bits", [P, I, I, I, I, P, P])
     decl("vlb_gemm_bias_residual_f32", [I, I, I, P, I, P, I, P, I, P, P, P, I, P])
     decl("vlb_dropout_bits_words", [L, I], L)

@@ -297,6 +297,18 @@ int vlb_mlm_ce_backward(void* logits_bf16, int ld, int V, const int32_t* lab, co
                         const float* gscale, void* stream) {
   COUNTED(1, mlm_ce_backward(logits_bf16, ld, V, lab, count, rows, lse, gscale, ST));
 }
+int vlb_soft_target_rows(const float* targets, int n, int C, int ld_t, int64_t* arg, void* stream) {
+  COUNTED(1, soft_target_rows(targets, n, C, ld_t, arg, ST));
+}
+int vlb_soft_ce_forward(const void* logits_bf16, int ld, int C, const float* targets, int ld_t, const int32_t* idx,
+                        const int32_t* lab, const int32_t* count, int rows, float* lse, float* row_loss, int32_t* correct,
+                        void* stream) {
+  COUNTED(1, soft_ce_forward(logits_bf16, ld, C, targets, ld_t, idx, lab, count, rows, lse, row_loss, correct, ST));
+}
+int vlb_soft_ce_backward(void* logits_bf16, int ld, int C, const float* targets, int ld_t, const int32_t* idx,
+                         const int32_t* count, int rows, const float* lse, const float* w, void* stream) {
+  COUNTED(1, soft_ce_backward(logits_bf16, ld, C, targets, ld_t, idx, count, rows, lse, w, ST));
+}
 int vlb_grad_sqnorm(const VlbAdamWTensor* descs_device, int count, float* sq, void* stream) {
   COUNTED(1, grad_sqnorm(descs_device, count, sq, ST));
 }

@@ -6,6 +6,10 @@
 // (label_compact_kernel), the transform + decoder GEMMs run on those rows only (the library GEMM), and the cross-entropy is one
 // pass over the bf16 logits (mlm_ce_forward_kernel: online log-sum-exp, label logit, arg-max for the accuracy metric) with the
 // gradient written in place by mlm_ce_backward_kernel.
+// The masked-region-classification loss of the same task (soft_cross_entropy, common/utils/misc.py:124-151, on the region
+// classifier VisualLinguisticBertMVRCHead, common/visual_linguistic_bert.py:473-502) follows the same plan: its valid rows
+// (target sum within 0.1 of 1) are found by soft_target_rows_kernel and compacted by label_compact_kernel, and the soft-target
+// cross-entropy reads the fp32 targets in place (soft_ce_forward_kernel / soft_ce_backward_kernel).
 #include "ops.cuh"
 
 namespace vlb {
@@ -167,6 +171,133 @@ mlm_ce_backward_kernel(__nv_bfloat16* __restrict__ logits, int ld, int V, const 
   }
 }
 
+// ---- masked visual region classification (MVRC) ---------------------------------------------------------------------------
+// soft_cross_entropy of common/utils/misc.py:124-151 on the regions whose fp32 target row sums to 1 +- 0.1.
+
+__device__ __forceinline__ void argmax_step(float v, int c, float& m, int& am) {
+  if (v > m) { m = v; am = c; }
+}
+
+// One warp per target row: arg[row] = first index of the row's maximum when |sum - 1| < 0.1, else -1 (the int64 label array
+// label_compact_kernel takes, with ignore = -1).  Rows are C fp32 at stride ld_t and only 4-byte aligned (C = 1601): the
+// unaligned head and the tail are read as scalars, the middle as float4.  Each lane sees its indices in ascending order, so
+// its strict '>' keeps the first maximum; the lane merge takes the smallest index among equal maxima.
+__global__ void __launch_bounds__(256)
+soft_target_rows_kernel(const float* __restrict__ t, int n, int C, int ld_t, int64_t* __restrict__ arg) {
+  pdl_trigger();
+  pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= n) return;
+  const float* __restrict__ tr = t + (size_t)row * ld_t;
+  const int head = min(C, (int)(((16u - (reinterpret_cast<uintptr_t>(tr) & 15u)) & 15u) >> 2));
+  const int nvec = (C - head) >> 2;
+  const int tail0 = head + (nvec << 2);
+  float s = 0.0f, m = -INFINITY;
+  int am = 0x7fffffff;
+  if (lane < head) {
+    const float v = __ldg(tr + lane);
+    s += v;
+    argmax_step(v, lane, m, am);
+  }
+  const float4* __restrict__ tv = reinterpret_cast<const float4*>(tr + head);
+  for (int v = lane; v < nvec; v += 32) {
+    const float4 q = __ldg(tv + v);
+    const int c = head + (v << 2);
+    s += (q.x + q.y) + (q.z + q.w);
+    argmax_step(q.x, c, m, am);
+    argmax_step(q.y, c + 1, m, am);
+    argmax_step(q.z, c + 2, m, am);
+    argmax_step(q.w, c + 3, m, am);
+  }
+  if (tail0 + lane < C) {
+    const float v = __ldg(tr + tail0 + lane);
+    s += v;
+    argmax_step(v, tail0 + lane, m, am);
+  }
+  s = warp_sum(s);
+  const float gm = warp_max(m);
+  int cand = (m == gm) ? am : 0x7fffffff;
+  for (int o = 16; o > 0; o >>= 1) cand = min(cand, __shfl_xor_sync(0xffffffffu, cand, o));
+  if (lane == 0) arg[row] = fabsf(s - 1.0f) < 0.1f ? (int64_t)cand : (int64_t)-1;
+}
+
+// One block per compacted row < count: the bf16 logits row (ld, padding columns biased to -30000) and the fp32 target row
+// targets[idx[row]] read in place.  lse[row] = log sum_c exp(x_c), row_loss[row] = S lse - sum_c t_c x_c
+// (= -sum_c t_c log_softmax(x)_c, S = sum_c t_c), correct += (logit arg-max == lab[row]).  Rows >= count: row_loss = 0.
+__global__ void __launch_bounds__(256)
+soft_ce_forward_kernel(const __nv_bfloat16* __restrict__ logits, int ld, int C, const float* __restrict__ targets, int ld_t,
+                       const int32_t* __restrict__ idx, const int32_t* __restrict__ lab, const int32_t* __restrict__ count,
+                       float* __restrict__ lse, float* __restrict__ row_loss, int32_t* __restrict__ correct) {
+  __shared__ float red[8];
+  __shared__ int redi[8];
+  pdl_trigger();
+  pdl_wait();
+  const int row = blockIdx.x;
+  if (row >= count[0]) {
+    if (threadIdx.x == 0) { row_loss[row] = 0.0f; lse[row] = 0.0f; }
+    return;
+  }
+  const __nv_bfloat16* __restrict__ lr = logits + (size_t)row * ld;
+  const float* __restrict__ tr = targets + (size_t)idx[row] * ld_t;
+  float m = -INFINITY, dot = 0.0f, s = 0.0f;
+  int am = 0x7fffffff;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const float x = __bfloat162float(lr[c]);
+    const float tc = __ldg(tr + c);
+    argmax_step(x, c, m, am);
+    dot = fmaf(tc, x, dot);
+    s += tc;
+  }
+  const float gmax = block_max(m, red);
+  int cand = (m == gmax) ? am : 0x7fffffff;
+  for (int o = 16; o > 0; o >>= 1) cand = min(cand, __shfl_xor_sync(0xffffffffu, cand, o));
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) redi[threadIdx.x >> 5] = cand;
+  __syncthreads();
+  int best = redi[0];
+  for (int w = 1; w < (int)(blockDim.x >> 5); ++w) best = min(best, redi[w]);
+  float e = 0.0f;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) e += __expf(__bfloat162float(lr[c]) - gmax);
+  const float tot = block_add(e, red);
+  const float dsum = block_add(dot, red);
+  const float ssum = block_add(s, red);
+  if (threadIdx.x == 0) {
+    const float l = gmax + __logf(tot);
+    lse[row] = l;
+    row_loss[row] = ssum * l - dsum;
+    if (best == lab[row]) atomicAdd(correct, 1);
+  }
+}
+
+// IN PLACE over the logits: d[row, c] = (S exp(x_c - lse[row]) - t_c) * w[row] for rows < count, c < C, with S the row's own
+// target sum (valid rows sum to anything in (0.9, 1.1)); 0 for rows >= count and the padding columns C .. ld-1.
+__global__ void __launch_bounds__(256)
+soft_ce_backward_kernel(__nv_bfloat16* __restrict__ logits, int ld, int C, const float* __restrict__ targets, int ld_t,
+                        const int32_t* __restrict__ idx, const int32_t* __restrict__ count, const float* __restrict__ lse,
+                        const float* __restrict__ w) {
+  __shared__ float red[8];
+  pdl_trigger();
+  pdl_wait();
+  const int row = blockIdx.x;
+  __nv_bfloat16* __restrict__ lr = logits + (size_t)row * ld;
+  if (row >= count[0]) {
+    const int nvec = ld >> 3;
+    for (int v = threadIdx.x; v < nvec; v += blockDim.x) *reinterpret_cast<uint4*>(lr + v * 8) = make_uint4(0u, 0u, 0u, 0u);
+    return;
+  }
+  const float* __restrict__ tr = targets + (size_t)idx[row] * ld_t;
+  float s = 0.0f;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) s += __ldg(tr + c);
+  const float S = block_add(s, red);
+  const float l = lse[row], wr = w[row];
+  for (int c = threadIdx.x; c < ld; c += blockDim.x) {
+    float d = 0.0f;
+    if (c < C) d = (S * __expf(__bfloat162float(lr[c]) - l) - __ldg(tr + c)) * wr;
+    lr[c] = __float2bfloat16_rn(d);
+  }
+}
+
 }  // namespace
 
 int label_compact(const int64_t* labels, int n, int64_t ignore_index, int32_t* idx, int32_t* lab, int cap, int32_t* count,
@@ -191,6 +322,30 @@ int mlm_ce_backward(void* logits, int ld, int V, const int32_t* lab, const int32
   VLB_REQUIRE(logits && lab && count && lse && gscale && rows > 0 && V > 0 && ld >= V && ld % 8 == 0, "mlm_ce_backward: bad arguments");
   VLB_CHECK_CUDA(launch_pdl(mlm_ce_backward_kernel, dim3(rows), dim3(256), 0, stream, static_cast<__nv_bfloat16*>(logits), ld, V, lab, count,
                             lse, gscale));
+  return VLB_OK;
+}
+
+int soft_target_rows(const float* targets, int n, int C, int ld_t, int64_t* arg, cudaStream_t stream) {
+  VLB_REQUIRE(targets && arg && n > 0 && C > 0 && ld_t >= C, "soft_target_rows: bad arguments (n=%d C=%d ld_t=%d)", n, C, ld_t);
+  VLB_CHECK_CUDA(launch_pdl(soft_target_rows_kernel, dim3((n + 7) / 8), dim3(256), 0, stream, targets, n, C, ld_t, arg));
+  return VLB_OK;
+}
+
+int soft_ce_forward(const void* logits, int ld, int C, const float* targets, int ld_t, const int32_t* idx, const int32_t* lab,
+                    const int32_t* count, int rows, float* lse, float* row_loss, int32_t* correct, cudaStream_t stream) {
+  VLB_REQUIRE(logits && targets && idx && lab && count && lse && row_loss && correct && rows > 0 && C > 0 && ld >= C && ld % 8 == 0 &&
+              ld_t >= C, "soft_ce_forward: bad arguments (rows=%d C=%d ld=%d ld_t=%d)", rows, C, ld, ld_t);
+  VLB_CHECK_CUDA(launch_pdl(soft_ce_forward_kernel, dim3(rows), dim3(256), 0, stream, static_cast<const __nv_bfloat16*>(logits), ld, C,
+                            targets, ld_t, idx, lab, count, lse, row_loss, correct));
+  return VLB_OK;
+}
+
+int soft_ce_backward(void* logits, int ld, int C, const float* targets, int ld_t, const int32_t* idx, const int32_t* count, int rows,
+                     const float* lse, const float* w, cudaStream_t stream) {
+  VLB_REQUIRE(logits && targets && idx && count && lse && w && rows > 0 && C > 0 && ld >= C && ld % 8 == 0 && ld_t >= C,
+              "soft_ce_backward: bad arguments (rows=%d C=%d ld=%d ld_t=%d)", rows, C, ld, ld_t);
+  VLB_CHECK_CUDA(launch_pdl(soft_ce_backward_kernel, dim3(rows), dim3(256), 0, stream, static_cast<__nv_bfloat16*>(logits), ld, C,
+                            targets, ld_t, idx, count, lse, w));
   return VLB_OK;
 }
 

@@ -75,6 +75,11 @@ int mlm_ce_forward(const void* logits, int ld, int V, const int32_t* lab, const 
                    int32_t* correct, cudaStream_t stream);
 int mlm_ce_backward(void* logits, int ld, int V, const int32_t* lab, const int32_t* count, int rows, const float* lse,
                     const float* gscale, cudaStream_t stream);
+int soft_target_rows(const float* targets, int n, int C, int ld_t, int64_t* arg, cudaStream_t stream);
+int soft_ce_forward(const void* logits, int ld, int C, const float* targets, int ld_t, const int32_t* idx, const int32_t* lab,
+                    const int32_t* count, int rows, float* lse, float* row_loss, int32_t* correct, cudaStream_t stream);
+int soft_ce_backward(void* logits, int ld, int C, const float* targets, int ld_t, const int32_t* idx, const int32_t* count, int rows,
+                     const float* lse, const float* w, cudaStream_t stream);
 
 int grad_sqnorm(const VlbAdamWTensor* descs_device, int count, float* sq, cudaStream_t stream);
 int adamw_step(const VlbAdamWTensor* descs_device, const float* hyper_device, int count, double beta1, double beta2, double eps,

@@ -800,6 +800,102 @@ class MLMLossFn(torch.autograd.Function):
         return d_text.view(B, T, H), None, d_tw, d_tb, d_ln_w, d_ln_b, d_w[:V], d_bias[:V], None, None
 
 
+class MVRCLossFn(torch.autograd.Function):
+    """Masked visual region classification loss of the pre-training task on the valid regions only (csrc/heads.cu):
+    forward(object_out f32 [B,R,H], mvrc_labels f32 [B,R,C] (soft targets), transform.dense.weight/bias,
+            region_cls_pred.weight [C,H] / bias [C], cap, norm_in_batch_first)
+      -> (loss, n_correct int32[1], n_valid int32[1])
+    i.e. soft_cross_entropy(VisualLinguisticBertMVRCHead(object_out).view(-1, C), mvrc_labels.view(-1, C)) of
+    pretrain/modules/resnet_vlbert_for_pretraining.py:191-203 without the logits of the other regions.  A region is valid when
+    its target row sums to 1 within 0.1 (common/utils/misc.py:133).
+      norm_in_batch_first False: loss = sum of row losses / rows used                       (reduction='mean')
+      norm_in_batch_first True : loss = sum_rows row_loss / (rows used in its sample + 1e-4), / (samples with a row + 1e-4)
+    `cap` = static upper bound of valid rows (rows the GEMMs run on).  When more rows are valid, the first `cap` (ascending
+    flat order) are used and the normalisation counts only those; n_valid still reports the true count.  No valid row:
+    loss 0 and all gradients 0."""
+
+    @staticmethod
+    def forward(ctx, object_out, mvrc_labels, tw, tb, cw, cb, cap, norm_in_batch_first):
+        _require_cuda(object_out, mvrc_labels, cw)
+        for nm, t in (("transform.dense.weight", tw), ("transform.dense.bias", tb), ("region_cls_pred.weight", cw),
+                      ("region_cls_pred.bias", cb)):
+            _require_param(t, "mvrc_head." + nm, object_out.device)
+        B, R, H = object_out.shape
+        n, C = B * R, cw.shape[0]
+        if tuple(mvrc_labels.shape) != (B, R, C):
+            raise RuntimeError("vlbert_b200: mvrc_labels must be [B, R, C] = %s (got %s)" % ((B, R, C), tuple(mvrc_labels.shape)))
+        Cp = (C + 7) // 8 * 8
+        cap = (int(cap) + 7) // 8 * 8
+        dev = object_out.device
+        lib, st = _lib.lib(), _stream()
+        i32 = torch.int32
+        tgt = mvrc_labels.contiguous().view(n, C).float()
+        arg = torch.empty((n,), dtype=torch.int64, device=dev)
+        _chk(lib.vlb_soft_target_rows(_p(tgt), n, C, C, _p(arg), st))
+        idx = torch.empty((cap,), dtype=i32, device=dev)
+        lab = torch.empty((cap,), dtype=i32, device=dev)
+        count = torch.empty((1,), dtype=i32, device=dev)
+        _chk(lib.vlb_label_compact(_p(arg), n, -1, _p(idx), _p(lab), cap, _p(count), st))
+        x16 = gather_rows(object_out.contiguous().view(n, H).float(), idx, cap, BF16)
+        tw16 = torch.empty((H, H), dtype=BF16, device=dev)
+        _chk(lib.vlb_cast_f32_to_bf16(_p(tw), _p(tw16), tw.numel(), st))
+        h = torch.empty((cap, H), dtype=BF16, device=dev)
+        z = torch.empty((cap, H), dtype=BF16, device=dev)
+        gemm(0, x16, tw16, h, bias=tb, act=1, aux=z)                         # dense + bias + erf-GELU (GELU' kept)
+        w16 = torch.zeros((Cp, H), dtype=BF16, device=dev)                   # classifier rows padded to 8
+        _chk(lib.vlb_cast_f32_to_bf16(_p(cw), _p(w16), cw.numel(), st))
+        bias_p = torch.full((Cp,), -30000.0, dtype=F32, device=dev)          # padding columns never win the softmax
+        bias_p[:C] = cb
+        logits = torch.empty((cap, Cp), dtype=BF16, device=dev)
+        gemm(0, h, w16, logits, bias=bias_p)
+        lse = torch.empty((cap,), dtype=F32, device=dev)
+        row_loss = torch.empty((cap,), dtype=F32, device=dev)
+        correct = torch.zeros((1,), dtype=i32, device=dev)
+        _chk(lib.vlb_soft_ce_forward(_p(logits), Cp, C, _p(tgt), C, _p(idx), _p(lab), _p(count), cap, _p(lse), _p(row_loss),
+                                     _p(correct), st))
+        # wrow[k] = d loss / d row_loss[k], on the device (rows beyond the rows used have row_loss 0 and get no gradient)
+        used = idx >= 0
+        if norm_in_batch_first:
+            sample = torch.where(used, idx // R, 0).long()
+            per_sample = torch.zeros((B,), dtype=F32, device=dev).index_add_(0, sample, used.to(F32))
+            n_has = (per_sample > 0).sum().to(F32)
+            wrow = used.to(F32) / ((per_sample[sample] + 1e-4) * (n_has + 1e-4))
+        else:
+            wrow = used.to(F32) / used.sum().clamp(min=1).to(F32)
+        loss = (row_loss * wrow).sum()
+        ctx.save_for_backward(x16, tw16, h, z, w16, logits, tgt, idx, count, lse, wrow)
+        ctx.dims = (B, R, H, C, Cp, cap)
+        ctx.mark_non_differentiable(correct, count)
+        return loss, correct, count
+
+    @staticmethod
+    def backward(ctx, g_loss, _gc, _gn):
+        x16, tw16, h, z, w16, logits, tgt, idx, count, lse, wrow = ctx.saved_tensors
+        B, R, H, C, Cp, cap = ctx.dims
+        dev = x16.device
+        lib, st = _lib.lib(), _stream()
+        w = (wrow * g_loss.detach().to(F32)).contiguous()
+        _chk(lib.vlb_soft_ce_backward(_p(logits), Cp, C, _p(tgt), C, _p(idx), _p(count), cap, _p(lse), _p(w), st))
+        dlog = logits                                                         # in place: d loss / d logits, bf16 [cap, Cp]
+        d_bias = torch.zeros((Cp,), dtype=F32, device=dev)
+        _chk(lib.vlb_colsum_bf16(_p(dlog), Cp, _p(d_bias), cap, Cp, st))
+        d_w = torch.zeros((Cp, H), dtype=F32, device=dev)
+        d_w._vlb_accumulate = True
+        gemm(2, dlog, h, d_w)                                                 # dW = dlogits^T h
+        d_pre = torch.empty((cap, H), dtype=BF16, device=dev)
+        gemm(1, dlog, w16, d_pre, act=3, aux=z)                               # (dlogits W) x GELU'(pre-activation)
+        d_tb = torch.zeros((H,), dtype=F32, device=dev)
+        _chk(lib.vlb_colsum_bf16(_p(d_pre), H, _p(d_tb), cap, H, st))
+        d_tw = torch.zeros((H, H), dtype=F32, device=dev)
+        d_tw._vlb_accumulate = True
+        gemm(2, d_pre, x16, d_tw)
+        dx = torch.empty((cap, H), dtype=BF16, device=dev)
+        gemm(1, d_pre, tw16, dx)
+        d_obj = torch.zeros((B * R, H), dtype=F32, device=dev)
+        scatter_rows_add(dx, idx, d_obj)
+        return d_obj.view(B, R, H), None, d_tw, d_tb, d_w[:C], d_bias[:C], None, None
+
+
 class GatherRowsFn(torch.autograd.Function):
     """out[i] = idx[i] >= 0 ? src[idx[i]] : 0 ; src 2-D (bf16 or f32) -> f32.  Each source row is referenced at most once."""
 

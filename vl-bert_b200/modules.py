@@ -472,6 +472,22 @@ class VisualLinguisticBertForPretraining(VisualLinguisticBert):
                                   p.transform.LayerNorm.weight, p.transform.LayerNorm.bias, p.decoder.weight, p.bias,
                                   int(max_labelled), 1e-12)
 
+    def mvrc_loss(self, object_out, mvrc_labels, max_valid=None, norm_in_batch_first=False):
+        """Fused masked-region-classification loss for callers that need the LOSS, not the [B, R, C] logits:
+        == soft_cross_entropy(self.mvrc_head(object_out).view(-1, C), mvrc_labels.view(-1, C)) (common/utils/misc.py:124-151,
+        pretrain/modules/resnet_vlbert_for_pretraining.py:191-203), or its MVRC_LOSS_NORM_IN_BATCH_FIRST form, evaluated on the
+        valid regions only (target row sum within 0.1 of 1): they are compacted on the device, the transform + classifier GEMMs
+        run on those rows, the soft-target cross-entropy is one pass over bf16 logits and the fp32 targets.
+        Returns (loss, n_correct, n_valid) -- n_correct counts what MVRCAccuracy counts (logit arg-max == target arg-max).
+        max_valid: static upper bound of valid regions (no host sync; CUDA-graph friendly); None = counted on the host.  If more
+        regions are valid than max_valid, the first max_valid (ascending flat order) are used and the loss is normalised by
+        the regions used (per sample in batch-first mode); n_valid reports the true count, so callers can detect it."""
+        h = self.mvrc_head
+        if max_valid is None:
+            max_valid = max(8, int(((mvrc_labels.sum(-1) - 1).abs() < 0.1).sum().item()))
+        return VF.MVRCLossFn.apply(object_out, mvrc_labels, h.transform.dense.weight, h.transform.dense.bias,
+                                   h.region_cls_pred.weight, h.region_cls_pred.bias, int(max_valid), bool(norm_in_batch_first))
+
 
 # ------------------------------------------------------------------------------------------------
 # region-feature front end
